@@ -2,7 +2,7 @@
 """bench.py -- decode tokens/s (bs=1) of a Llama-2-7B-shaped EXL2 ~4.0 bpw model on the B200-native hot path,
 with the q_gemm path's achieved HBM GB/s against the measured roofline.  BASELINE.json metric / configs[2].
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model PRESET]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model PRESET] [--dump-outputs DIR]
 
 A "step" is one decode token: embedding -> 32 x (Q4-KV unpack, RMSNorm+QKV+RoPE, paged attention, Q4-KV pack,
 O-proj+residual, RMSNorm+gate|up+silu*mul, down+residual) -> RMSNorm -> lm_head.  Weights are synthetic tensors in the
@@ -18,6 +18,10 @@ JSON keys (one line on stdout):
   cpu_baseline          oracle/exl2_cpu.c (the CPU port of the reference's q_gemm) on the host cores, bounded sample
   --impl reference      the CPU arm alone (the reference has no CPU q_gemm; its CUDA extension is timed separately by
                         tools/microbench.py --ref and reported under "reference_cuda_ext" when oracle/_ref is present)
+
+--dump-outputs DIR writes what the timed path computed in its last timed step as DIR/<name>.npy (float32): for decode the
+logits [1, vocab] and the greedy next token [1, 1], for --mode prefill the hidden state [16, T, hidden].  Weights, prompt
+and synthetic context are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -31,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it
 
 METRIC = "decode tokens/sec (bs=1) Llama2-7B EXL2-4.0bpw"       # the default --model; other presets are named in config.workload
 UNIT = "tokens/s"
@@ -48,6 +53,23 @@ def measured_peaks() -> tuple[float, str]:
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+DUMP_LIMIT = 64 * 10**6          # bytes of all .npy files of one --dump-outputs, headers included
+
+
+def dump_outputs(path: str, tensors: dict) -> None:
+    """Save each tensor as <path>/<name>.npy in float32.  Past DUMP_LIMIT bytes in all, an array larger than its even share
+    is replaced by a fixed, seeded sample of its flattened elements (same indices on every run)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = (DUMP_LIMIT // len(tensors) - 4096) // 4          # elements; 4096 bytes left for the .npy header
+    for name, t in tensors.items():
+        a = t.detach().float().cpu().numpy()
+        if a.size > share and sum(x.numel() for x in tensors.values()) > share * len(tensors):
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -286,6 +308,8 @@ def run_ours(args, rank, world):
     ms_per_step = ms_total / K
     assert bool(torch.isfinite(dec.logits).all()), "decode produced non-finite logits"
     value = 1000.0 / ms_per_step
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": dec.logits, "next_token": dec.ids})
 
     # ---- parity of the TIMED path: the same token through the chained launches (what the graph replays) and through the
     #      reference's un-chained op sequence (q_attn_forward_1 incl. rope_, attention, q_attn_forward_2, q_mlp_forward_, rms_norm
@@ -441,7 +465,9 @@ def run_prefill(args):
             if i:
                 ts.append(e0.elapsed_time(e1))
         return sorted(ts)[len(ts) // 2], out
-    ms_rows, x_rows = timed(dec.prefill_rows, max(2, min(args.steps, 8)))
+    ms_rows, x_rows = timed(dec.prefill_rows, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"hidden": x_rows})
     ms_chunk, x_chunk = timed(lambda p: dec.prefill(p, chunk=8), 1)
     # same prompt, two schedules: the hidden state of the last chunk must agree (Q4 cache in the loop: loose tolerance)
     a, b = x_rows[:, -8:].float(), x_chunk.float()
@@ -472,7 +498,13 @@ def main():
     ap.add_argument("--mode", default="decode", choices=["decode", "prefill"])
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-ref-ext", action="store_true", help="skip the reference-extension leg (oracle/_ref on the same GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":

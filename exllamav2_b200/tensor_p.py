@@ -332,6 +332,8 @@ def run_bench(args, rank: int, world: int, metric: str, unit: str):
     dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_per_step = float(ms.item()) / K
     finite = bool(torch.isfinite(dec.logits).all())
+    if rank == 0 and args.dump_outputs:
+        bench_mod.dump_outputs(args.dump_outputs, {"logits": dec.logits, "next_token": dec.ids})
 
     # e2e: host token in, host logits out, every step (rank 0's host feeds all ranks through a broadcast of the id)
     ids_host = torch.zeros((1, 1), dtype=torch.long).pin_memory()

@@ -48,3 +48,31 @@ def activations(name, M, seed=0):
 
 def u16(x):
     return np.ascontiguousarray(x).view(np.uint16)
+
+
+# cases compared with the reference extension's outputs stored in golden/reference_parity.npz (oracle/gen_golden.py)
+REF_GEMM_M = (1, 4, 8, 19)
+
+
+def ref_cases():
+    """The linear cases the reference's kernels support (N a multiple of 32)."""
+    return [n for n in list(EXL2_CASES) + list(GPTQ_CASES) if case_shape(n)[1] % 32 == 0]
+
+
+def ref_ops_inputs():
+    """Seeded inputs of the rms_norm / rope / Q4-kv comparison with the reference, in their draw order."""
+    rng = np.random.default_rng(123)
+    d = {"norm_x": rng.normal(0, 1.5, size=(5, 4096)).astype(np.float16),
+         "norm_w": (1 + 0.1 * rng.normal(size=(4096,))).astype(np.float16)}
+    for tag in ("neox", "gptj"):
+        d[f"rope_{tag}_x"] = rng.normal(0, 1, size=(2, 6, 8 * 128)).astype(np.float16)
+    d["kv_k"] = rng.normal(0, 1, size=(2, 9, 8, 128)).astype(np.float16)
+    d["kv_v"] = rng.normal(0, 3, size=(2, 9, 8, 128)).astype(np.float16)
+    return d
+
+
+def gptq_4096_row(act_order):
+    """BASELINE config 1: a GPTQ 4096 x 4096 g128 matrix and one activation row."""
+    w = synth.make_gptq(4096, 4096, 128, seed=0, act_order=act_order)
+    a = np.random.default_rng(0).normal(0, 1, size=(1, 4096)).astype(np.float16)
+    return w, a
